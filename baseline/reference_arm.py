@@ -1,13 +1,13 @@
 """The one part of the reference that builds in this image, run UNMODIFIED: its OpenMP concurrency bench.
 
-argonne-lcf/HPC-Patterns has no Python package (``pip install /root/reference`` -> "not installable: neither
-setup.py nor pyproject.toml"), its GPU programs need icpx/SYCL, Level-Zero and a GPU-aware MPICH, none of which
-exist here — so the GPU headline has no reference arm (``bench.py --impl reference`` says so).  What does build
-is BASELINE.json's config #1, "concurency/bench compute+copy overlap on CPU host (OpenMP, no GPU)":
-``concurency/main.cpp`` + ``concurency/bench_omp.cpp`` with plain ``g++ -fopenmp`` (target regions fall back
-to the host).  ``baseline/_ref`` is a verbatim copy of ``/root/reference`` (git-ignored, travels to the GPU box);
-the only build-line addition is ``-Domp_target_alloc_host=omp_target_alloc`` (an Intel extension mapped to the
-standard call on the command line; the sources are untouched), the same two builds as concurency/run_omp.sh:6-7.
+argonne-lcf/HPC-Patterns has no Python package (no setup.py nor pyproject.toml), its GPU programs need icpx/SYCL,
+Level-Zero and a GPU-aware MPICH, none of which a CUDA machine has — so the GPU headline has no reference arm
+(``bench.py --impl reference`` says so).  What does build is BASELINE.json's config #1, "concurency/bench
+compute+copy overlap on CPU host (OpenMP, no GPU)": ``concurency/main.cpp`` + ``concurency/bench_omp.cpp`` with plain
+``g++ -fopenmp``, compiled from an unmodified checkout (HPCP_REFERENCE) into ``oracle/_ref`` by oracle/reference_omp.py
+(``__graft_entry__.build()`` runs it when HPCP_REFERENCE is set; the binaries are git-ignored).  The run of the
+reference's nowait build on ``concurency_args()`` is recorded in tests/golden/ (oracle/make_golden.py), so the tests
+check this arm against it where no build of the reference exists.
 
 Both arms run the reference's five command groups (run_omp.sh:9) through each program's stock ``main()`` and
 report the same numbers, parsed from the same stdout contract (main.cpp:284-319).
@@ -17,47 +17,45 @@ from __future__ import annotations
 import math
 import os
 import re
-import shutil
 import subprocess
 from typing import Dict, List, Optional
 
+from oracle import reference_omp
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
-REF_SRC = os.environ.get("HPCP_REFERENCE", "/root/reference")
 GROUPS = ["C C", "C M2D", "C D2M", "M2D D2M", "H2D D2H"]          # concurency/run_omp.sh:9
-MODES = {"nowait": "NOWAIT", "host_threads": "HOST_THREADS"}       # run_omp.sh:6-7
-
-
-def host_cxx() -> str:
-    return os.environ.get("HOSTCXX") or ("/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++")
-
-
-def ensure_ref() -> Optional[str]:
-    """Verbatim copy of the reference under baseline/_ref (made once, where /root/reference is mounted)."""
-    if os.path.exists(os.path.join(REF_DIR, "concurency", "main.cpp")):
-        return REF_DIR
-    if not os.path.exists(os.path.join(REF_SRC, "concurency", "main.cpp")):
-        return None
-    if os.path.isdir(REF_DIR):
-        shutil.rmtree(REF_DIR)
-    shutil.copytree(REF_SRC, REF_DIR)
-    return REF_DIR
+MODES = reference_omp.MODES                                        # run_omp.sh:6-7
 
 
 def build_reference(mode: str = "nowait") -> Optional[str]:
-    ref = ensure_ref()
-    if ref is None or mode not in MODES:
+    """The reference's bench for `mode`: from HPCP_REFERENCE_BIN (a directory of prebuilt omp_<mode>) if set, else
+    built by build() into oracle/_ref, or built now from HPCP_REFERENCE."""
+    if mode not in MODES:
         return None
-    out_dir = os.path.join(ref, "_build")
-    exe = os.path.join(out_dir, f"omp_{mode}")
-    srcs = [os.path.join(ref, "concurency", f) for f in ("main.cpp", "bench_omp.cpp")]
-    if os.path.exists(exe) and all(os.path.getmtime(exe) >= os.path.getmtime(s) for s in srcs):
-        return exe
-    os.makedirs(out_dir, exist_ok=True)
-    p = subprocess.run([host_cxx(), "-O2", "-std=c++17", "-fopenmp", f"-D{MODES[mode]}",
-                        "-Domp_target_alloc_host=omp_target_alloc", *srcs, "-o", exe],
-                       capture_output=True, text=True, timeout=900)
-    return exe if p.returncode == 0 else None
+    if os.environ.get("HPCP_REFERENCE_BIN"):
+        exe = reference_omp.binary(mode, os.environ["HPCP_REFERENCE_BIN"])
+        return exe if os.path.exists(exe) else None
+    exe = reference_omp.binary(mode)
+    if not os.path.exists(exe):
+        tree = reference_omp.reference_tree()
+        if tree is None:
+            return None
+        try:
+            reference_omp.build(tree)
+        except (OSError, subprocess.SubprocessError):
+            return None
+    return exe
+
+
+def concurency_args(mode: str = "nowait", repetitions: int = 5, elements: int = 8_000_000,
+                    tripcount: int = 40000) -> List[str]:
+    """The command line (after the program name) both arms run: the five groups, every size given explicitly."""
+    args = [mode, "--repetitions", str(repetitions), "--tripcount_C", str(tripcount)]
+    for c in ("MD", "DM", "HD", "DH"):
+        args += [f"--globalsize_{c}", str(elements)]
+    for g in GROUPS:
+        args += ["--commands"] + g.split()
+    return args
 
 
 def ours_binary() -> Optional[str]:
@@ -113,11 +111,7 @@ def run_cpu_concurency(impl: str, mode: str = "nowait", repetitions: int = 5, el
     exe = build_reference(mode) if impl == "reference" else ours_binary()
     if exe is None:
         return {"impl": impl, "unavailable": "reference tree / binary not present"}
-    cmd = [exe, mode, "--repetitions", str(repetitions), "--tripcount_C", str(tripcount)]
-    for c in ("MD", "DM", "HD", "DH"):
-        cmd += [f"--globalsize_{c}", str(elements)]
-    for g in GROUPS:
-        cmd += ["--commands"] + g.split()
+    cmd = [exe] + concurency_args(mode, repetitions, elements, tripcount)
     env = dict(os.environ)
     env["OMP_NUM_THREADS"] = str(threads or min(os.cpu_count() or 1, 8))
     env.pop("OMP_PROC_BIND", None)

@@ -14,7 +14,8 @@ buffers), K steps are ONE persistent launch, no NCCL / cudaMemcpy / host sync on
 message to (or from) each neighbour: value = N x 2 x message / time.  `rows` balances the step's HBM time against its
 NVLink time, the rule of the reference's autotuner (concurency/main.cpp:219-258).  N=1: the rank is its own neighbour.
 
-Contract: `python bench.py --gpus N --steps K --warmup W`; for N>1 launched by torchrun (one rank per GPU).
+Contract: `python bench.py --gpus N --steps K --warmup W [--dump-outputs DIR]`; for N>1 launched by torchrun (one rank
+per GPU).  `--dump-outputs` writes the field the timed call computes (see dump_field) for comparing two builds.
 Rank 0 prints ONE JSON line.  Timing: W>=3 untimed warm-up steps, a time-based pre-heat, then `--blocks` blocks of
 EXACTLY K steps, each behind an in-kernel cross-GPU barrier, CUDA events on the launching stream, max over ranks;
 `value` is the best block (the reference reports the minimum over 10 iterations, peer2pear.cpp:23,52), all blocks are
@@ -79,7 +80,42 @@ def parse_args():
     ap.add_argument("--preheat-ms", type=float, default=float(os.environ.get("HPCP_BENCH_PREHEAT_MS", "300")))
     ap.add_argument("--e2e-steps", type=int, default=4)
     ap.add_argument("--no-extras", action="store_true", help="skip the unfused / stock / legacy comparison runs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the field the timed call computes as DIR/field_rank<r>.npy "
+                         "(float32, a fixed sample of columns when larger than DUMP_ELEMS over all ranks)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.blocks < 1:
+        ap.error("--steps and --blocks must be >= 1")
+    return args
+
+
+DUMP_ELEMS = 8 << 20        # float32 words over all ranks: 32 MB per dump
+
+
+def dump_columns(row_elems: int, ncols: int):
+    """The columns a dump keeps: the same ones in every run with the same --bytes / --gpus (seeded, sorted)."""
+    import numpy as np
+
+    if ncols >= row_elems:
+        return None
+    return np.sort(np.random.default_rng(0).choice(row_elems, ncols, replace=False))
+
+
+def dump_field(hs, steps: int, out_dir: str) -> None:
+    """What a caller of the timed path receives: this rank's slab after one ``hs.step(steps)`` call.  The call is
+    replayed from the closed-form initial field (reset()), because how many steps the timed series ran depends on the
+    time-based pre-heat; so runs with the same arguments get the same input and two builds compare word for word."""
+    import numpy as np
+    import torch
+
+    hs.reset()
+    hs.step(steps)
+    u = hs.u_tensor()
+    cols = dump_columns(hs.row_elems, max(1, DUMP_ELEMS // hs.world // hs.rows))
+    if cols is not None:
+        u = u[:, torch.from_numpy(cols).to(u.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"field_rank{hs.rank}.npy"), u.cpu().numpy())
 
 
 def cpu_concurency(impl: str) -> dict:
@@ -155,6 +191,8 @@ def main() -> int:
                                         # barrier is enqueued before the start event, i.e. outside the region)
     total_fused_launches = hs.launches - launches0
     wrong_last = int(comm.sum(hs.verify_last_step()))
+    if args.dump_outputs:
+        dump_field(hs, K, args.dump_outputs)
     ms_per_step = fused["ms"]
     msg = args.bytes
     value = world * 2 * msg / (ms_per_step * 1e-3) / 1e9          # aggregate GB/s over all GPUs, both neighbours

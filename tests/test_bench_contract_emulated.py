@@ -72,6 +72,40 @@ def test_bench_line_has_the_contract_keys(emu, monkeypatch, capsys, extras):  # 
     assert not emu.live, "bench.py returned every allocation"
 
 
+def test_bench_dump_outputs_is_the_timed_call(emu, monkeypatch, capsys, tmp_path):  # noqa: F811
+    """--dump-outputs: the slab after one timed call (K steps from the initial field), the same whatever the pre-heat
+    and block count ran before it, equal to the PyTorch reference; a field larger than DUMP_ELEMS keeps its seeded
+    columns."""
+    import numpy as np
+
+    from hpc_patterns_b200.models.halo import initial_field, reference_steps
+
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: True)
+    monkeypatch.setattr(torch.cuda, "Event", TickingEvent)
+    for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK", "HPCP_DEVICE"):
+        monkeypatch.delenv(k, raising=False)
+    msg, steps = 8192, 5
+    want = reference_steps(initial_field(1, 8, msg // 4), steps).numpy()
+    dumps = []
+    for blocks, dump_elems in ((3, None), (2, None), (2, 8 * 300)):
+        out = tmp_path / f"dump{len(dumps)}"
+        monkeypatch.setattr(sys, "argv", ["bench.py", "--gpus", "1", "--steps", str(steps), "--warmup", "3", "--bytes",
+                                          str(msg), "--tile-kb", "1", "--preheat-ms", "1", "--blocks", str(blocks),
+                                          "--e2e-steps", "1", "--no-extras", "--dump-outputs", str(out)])
+        bench = _load_bench()
+        if dump_elems:
+            monkeypatch.setattr(bench, "DUMP_ELEMS", dump_elems)
+        assert bench.main() == 0
+        assert [p.name for p in out.iterdir()] == ["field_rank0.npy"]
+        dumps.append(np.load(out / "field_rank0.npy"))
+    capsys.readouterr()
+    assert dumps[0].dtype == np.float32 and dumps[0].shape == (8, msg // 4)
+    assert np.array_equal(dumps[0], want) and np.array_equal(dumps[1], want)
+    cols = bench.dump_columns(msg // 4, 300)
+    assert len(cols) == 300 and np.array_equal(dumps[2], want[:, cols])
+    assert not emu.live
+
+
 def test_reference_arm_line(monkeypatch, capsys):
     monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--gpus", "4", "--steps", "20", "--warmup", "5"])
     monkeypatch.delenv("RANK", raising=False)

@@ -110,37 +110,56 @@ def test_step_word_protocol_model(world, ctas, mode):
     assert all(v == steps for v in flags.values())
 
 
-def test_bench_reference_arm_prints_unavailable_and_cpu_numbers():
+# Stand-in for the reference's nowait build where none exists: it accepts only the command line the reference arm was
+# recorded with (tests/golden, oracle/make_golden.py) and replays that run's stdout and exit status.
+_REPLAY = """import gzip, json, sys
+rec = json.load(gzip.open({golden!r}, "rt"))["cpu_concurency"]
+if sys.argv[1:] != rec["argv"]:
+    sys.exit("not the recorded command line: %r" % sys.argv[1:])
+sys.stdout.write(rec["stdout"])
+sys.exit(rec["rc"])
+"""
+
+
+def _reference_arm_env(tmp_path):
+    """Environment for bench.py's reference arm and the binary it must report: the reference's own build when there
+    is one (HPCP_REFERENCE_BIN, oracle/_ref or HPCP_REFERENCE), else the recorded run."""
+    from oracle import reference_omp
+
+    env = dict(os.environ)
+    if env.get("HPCP_REFERENCE_BIN"):
+        return env, reference_omp.binary("nowait", env["HPCP_REFERENCE_BIN"])
+    if os.path.exists(reference_omp.binary("nowait")) or reference_omp.reference_tree() is not None:
+        return env, reference_omp.binary("nowait")
+    stand_in = tmp_path / "omp_nowait"
+    stand_in.write_text(f"#!{sys.executable}\n" +
+                        _REPLAY.format(golden=os.path.join(ROOT, "tests", "golden", "reference_concurency.json.gz")))
+    stand_in.chmod(0o755)
+    env["HPCP_REFERENCE_BIN"] = str(tmp_path)
+    return env, str(stand_in)
+
+
+def test_bench_reference_arm_prints_unavailable_and_cpu_numbers(tmp_path):
+    env, exe = _reference_arm_env(tmp_path)
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "1", "--steps", "2",
-                        "--warmup", "1"], capture_output=True, text=True, timeout=900)
+                        "--warmup", "1"], capture_output=True, text=True, timeout=900, env=env)
     assert p.returncode == 0, p.stderr[-2000:]
     d = json.loads(p.stdout.strip().splitlines()[-1])
     assert d["impl"] == "reference" and "unavailable" in d
-    if os.path.exists(os.path.join(ROOT, "baseline", "_ref", "concurency", "main.cpp")) or os.path.exists("/root/reference"):
-        cc = d["cpu_concurency"]
-        assert cc["impl"] == "reference" and cc["config"] == "cpu_concurency" and cc["groups"] == 5
-        assert cc["binary"].startswith("baseline/_ref/")
+    cc = d["cpu_concurency"]
+    assert cc["impl"] == "reference" and cc["config"] == "cpu_concurency" and cc["groups"] == 5, cc
+    assert cc["binary"] == os.path.relpath(exe, ROOT)
 
 
 @pytest.mark.parametrize("impl", ["reference", "ours"])
-def test_bench_cpu_concurency_config(impl, bin_dir):
-    if impl == "reference" and not (os.path.exists("/root/reference") or
-                                    os.path.exists(os.path.join(ROOT, "baseline", "_ref", "concurency"))):
-        pytest.skip("reference tree not present")
+def test_bench_cpu_concurency_config(impl, bin_dir, tmp_path):
+    env = _reference_arm_env(tmp_path)[0] if impl == "reference" else None
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", impl, "--config", "cpu_concurency"],
-                       capture_output=True, text=True, timeout=900)
+                       capture_output=True, text=True, timeout=900, env=env)
     assert p.returncode == 0, p.stderr[-2000:]
     d = json.loads(p.stdout.strip().splitlines()[-1])
-    assert d["impl"] == impl and d["value"] is not None and d["value"] > 0
+    assert d["impl"] == impl and d["value"] is not None and d["value"] > 0, d
     assert [g["commands"] for g in d["per_group"]] == ["C C", "C MD", "C DM", "MD DM", "HD DH"]
-
-
-def test_reference_copy_is_verbatim():
-    ref, src = os.path.join(ROOT, "baseline", "_ref"), "/root/reference"
-    if not (os.path.isdir(ref) and os.path.isdir(src)):
-        pytest.skip("needs both the mount and the copy")
-    for rel in ("concurency/main.cpp", "concurency/bench_omp.cpp", "concurency/bench.hpp", "p2p/peer2pear.cpp"):
-        assert open(os.path.join(ref, rel), "rb").read() == open(os.path.join(src, rel), "rb").read(), rel
 
 
 def test_block_timer_preheat_count_is_rank_independent():
