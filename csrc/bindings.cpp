@@ -77,6 +77,7 @@ HaloTuning halo_tuning_from(const py::dict& d) {
   if (d.contains("tile_kb")) t.tile_kb = d["tile_kb"].cast<int>();
   if (d.contains("stages")) t.stages = d["stages"].cast<int>();
   if (d.contains("l2_hint")) t.l2_hint = d["l2_hint"].cast<int>();
+  if (d.contains("depth")) t.depth = d["depth"].cast<int>();
   return t;
 }
 
@@ -318,6 +319,16 @@ PYBIND11_MODULE(_C, m) {
   m.attr("HALO_FLAG_BYTES") = static_cast<size_t>(kHaloFlagBytes);
   m.attr("HALO_FLAG_SETS") = kHaloFlagSets;
   m.attr("HALO_MAX_CTAS") = kHaloMaxCtas;
+  m.attr("HALO_DEFAULT_DEPTH") = kHaloDefaultDepth;
+  m.def(
+      "halo_sweep_depth",
+      [](int rows, const std::string& mode, const py::dict& tune) {
+        return halo_sweep_depth(rows, halo_mode_from(mode), halo_tuning_from(tune));
+      },
+      py::arg("rows"), py::arg("mode") = "pull", py::arg("tune") = py::dict(),
+      "Deepest sweep (steps per pass over the slab) a multi-step launch takes with these settings.");
+  m.def("halo_sweep_schedule", &halo_sweep_schedule, py::arg("steps"), py::arg("depth"),
+        "Sweep sizes of a `steps`-step launch whose deepest sweep is `depth`.");
   m.def(
       "halo_stencil_ctas",
       [](size_t row_elems, const std::string& mode, const py::dict& tune, int device) {

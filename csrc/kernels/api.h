@@ -15,6 +15,8 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <vector>
+
 namespace hpcp {
 
 constexpr int kApiMaxRanks = 16;
@@ -120,7 +122,10 @@ struct HaloTuning {
   int tile_kb = 0;  // bytes of a row per shared-memory stage in KiB; 0 -> 16
   int stages = 0;   // shared-memory stages (>= 6); 0 -> 6 (two CTAs per SM with 16 KiB tiles)
   int l2_hint = 0;  // 1: L2 evict_first policy on the streaming loads / stores of the slab's own rows
+  int depth = 0;    // pull: most steps one sweep of the slab may advance (deep halos); 0 -> kHaloDefaultDepth, 1 -> one
+                    // step per sweep (halo_stencil_kernel only)
 };
+constexpr int kHaloDefaultDepth = 3;  // measured: see docs/halo.md, "Deep sweeps"
 struct HaloStencilArgs {
   float* u[2] = {nullptr, nullptr};                 // local field, ping-pong: step g reads u[g&1], writes u[(g+1)&1]
   const float* left_u[2] = {nullptr, nullptr};      // pull: the left / right neighbour's u[0], u[1] (peer-mapped)
@@ -144,6 +149,11 @@ struct HaloStencilArgs {
 };
 // CTAs a launch with this geometry uses (identical on every rank; the flag words are indexed by it).
 int halo_stencil_ctas(size_t row_elems, const HaloTuning& tune, HaloMode mode, int device);
+// Deepest sweep a multi-step launch takes with these settings (1: every step is its own sweep).
+int halo_sweep_depth(int rows, HaloMode mode, const HaloTuning& tune);
+// Sweep sizes of a `steps`-step launch with maximum depth `depth`: greedy, the largest odd size <= min(depth, remaining
+// - 1), so every sweep is odd and the last one is a single step (identical on every rank).
+std::vector<int> halo_sweep_schedule(int steps, int depth);
 int launch_halo_stencil(const HaloStencilArgs& args, HaloMode mode, const HaloTuning& tune, int device,
                         cudaStream_t stream);
 // u[r][j] = u0(rank*rows + r, j); halo_lo / halo_hi (may be null) = the neighbours' boundary rows of the initial field.

@@ -269,6 +269,238 @@ __global__ void __launch_bounds__(kHaloThreads) halo_stencil_kernel(const HaloPa
   }
 }
 
+// ------------------------------------------------------------------ deep sweeps ----
+// halo_sweep_kernel<D> (pull only): one pass over the slab advances a column tile by up to D steps.  Columns are
+// independent and CTA c owns the same column tiles on every rank in every step, so a sweep of depth d starting at step
+// g loads the R + 2d input tiles of a column (rows -d .. R+d-1 of u[g&1]: the left neighbour's last d rows, its own R
+// rows, the right neighbour's first d rows), keeps the intermediate time levels on chip and stores only level d of rows
+// 0 .. R-1 into u[(g+d)&1].  HBM traffic per step falls from ~2R rows to ~2R/d; NVLink bytes per step stay the same.
+//
+// Schedule (halo_sweep_schedule, identical on every rank): greedy sweeps of the largest ODD size <= min(D, remaining-1),
+// so u[(g+d)&1] = u[(g+1)&1] keeps every parity-addressed buffer of the single-step kernel right, and the launch ends
+// with a one-step sweep: u[(g-1)&1] holds step g-1 afterwards, what verify_last_step() recomputes from.  The step words
+// are those of halo_stencil_kernel: wait for both neighbour words >= g at the start of a sweep, publish g+d at its end.
+// RAW: the neighbours' rows of step g are complete.  WAR: u[(g+d)&1] was last read by the neighbours' previous sweep
+// (odd length, same boundaries on every rank), which ended at g.
+//
+// On-chip wavefront.  Input tile i of a column (row m = i - d) arrives; for i >= 2 the math warps compute level 1 at
+// row m-1 from the three input tiles i-2, i-1, i (read from shared memory), then level L at row m-L from level L-1's
+// rows m-L-1, m-L (registers) and m-L+1 (just computed), L = 2 .. d.  Level L is valid from arrival 2L on, so arrivals
+// 2d .. R+2d-1 produce level d of rows 0 .. R-1, written IN PLACE over input tile i-2 (read only by this arrival and the
+// two before it).  Every thread owns fixed float4 positions of the tile: levels 1 .. D-1 keep two rows each in
+// registers.  Every arrival i >= 2 is one `computed` event of its slot i-2, stored or not.
+//
+// Slot rules (Ring cursors, S stages):
+//   * loads: tiles of a column in consecutive slots, R + 2d per column, at most S ahead of `retired`;
+//   * events: slot i-2 for arrival i = 2 .. R+2d-1; the cursor moves by 1 per event and by 2 more at the end of a
+//     column (the last two input tiles are never an event slot): +3 from the last event of a column to the next column's
+//     first, as in halo_stencil_kernel;
+//   * a stored event (i >= 2d) frees the tiles below it once bulk_wait_read<1> says the older stores have read their
+//     slots (`retired = t`, as halo_stencil_kernel); an unstored event (i < 2d, the first 2d-2 of a column) frees its
+//     own tile too, after bulk_wait_read<0> if a store is still pending (`retired = t + 1`) -- without that, the 2d + 1
+//     tiles a column needs before its first store would not fit a 6-slot ring for d >= 3.
+// tests/test_halo_sweep.py runs these rules as an executable model.
+// Three math warps: 4 warps per CTA, two CTAs = 2 warps per SM sub-partition, which leaves each thread up to 255
+// registers for the 2 x (D-1) x 11 float4 of wavefront state (D = 3: 247, no spills).  Eight math warps (9 warps per CTA,
+// up to 5 per sub-partition) cap a thread at 96 registers and spill.
+constexpr int kSweepMathWarps = 3;
+constexpr int kSweepThreads = 32 * (1 + kSweepMathWarps);
+constexpr uint32_t kSweepMaxTileBytes = 16 * 1024;  // register state is sized for 16 KiB tiles
+
+struct SweepParams {
+  unsigned char* u[2];
+  const unsigned char* left_u[2];   // the left neighbour's u[p] (row 0); a sweep of depth d pulls its rows R-d .. R-1
+  const unsigned char* right_u[2];  // the right neighbour's u[p]; a sweep of depth d pulls its rows 0 .. d-1
+  const uint32_t* wait_lo;
+  const uint32_t* wait_hi;
+  uint32_t* signal_lo;
+  uint32_t* signal_hi;
+  int rows;
+  size_t row_bytes;
+  size_t tile_begin, tile_end;
+  uint32_t tile_bytes;
+  int stages;
+  float alpha, s;
+  uint32_t step_base;
+  int steps;
+  uint64_t timeout_ns;
+  uint32_t* status;
+};
+
+__host__ __device__ __forceinline__ int sweep_depth(int remaining, int D) {
+  const int x = remaining - 1 < D ? remaining - 1 : D;
+  return x <= 1 ? 1 : x - 1 + (x & 1);  // largest odd <= x
+}
+
+template <int D>
+__global__ void __launch_bounds__(kSweepThreads, 2) halo_sweep_kernel(const SweepParams p) {
+  static_assert(D >= 3 && (D & 1) == 1, "deep sweeps have odd depth >= 3");
+  extern __shared__ __align__(128) unsigned char smem[];
+  const uint32_t T = p.tile_bytes;
+  const int S = p.stages;
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + static_cast<size_t>(S) * T);
+  uint64_t* computed = full + S;
+  volatile int* abort_w = reinterpret_cast<volatile int*>(computed + S);
+
+  if (threadIdx.x == 0) {
+    for (int i = 0; i < S; ++i) {
+      ptx::mbar_init(&full[i], 1);
+      ptx::mbar_init(&computed[i], kSweepMathWarps);
+    }
+    *abort_w = 0;
+    ptx::fence_mbar_init();
+  }
+  __syncthreads();
+
+  const int R = p.rows;
+  const size_t n_tiles = p.tile_end - p.tile_begin;
+  const size_t ncols = n_tiles > blockIdx.x ? (n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+  if (ncols == 0) return;  // same geometry on every rank: nobody waits for this CTA index
+  auto col_off = [&](size_t jj) { return (p.tile_begin + blockIdx.x + jj * gridDim.x) * static_cast<size_t>(T); };
+  auto col_len = [&](size_t off) {
+    return static_cast<uint32_t>(p.row_bytes - off < T ? p.row_bytes - off : T);
+  };
+
+  const int warp = threadIdx.x >> 5;
+  if (warp == 0) {
+    if (threadIdx.x != 0) return;
+    // ------------------------------------------------------------------ DMA thread ----
+    Ring ld{0, 0};    // next tile to load
+    Ring ev{0, 0};    // slot of the next event (input tile i-2 of arrival i)
+    Ring done{0, 0};  // next `computed` barrier to consume
+    for (int k = 0; k < p.steps;) {
+      const int d = sweep_depth(p.steps - k, D);
+      const uint32_t g = p.step_base + static_cast<uint32_t>(k);
+      const int in = static_cast<int>(g & 1u), out = in ^ 1;  // d is odd
+      const bool ok = wait_epoch(p.wait_lo + blockIdx.x * kHaloFlagWords, g, p.timeout_ns, p.status) &&
+                      wait_epoch(p.wait_hi + blockIdx.x * kHaloFlagWords, g, p.timeout_ns, p.status);
+      if (!ok) {
+        *abort_w = 1;
+        return;
+      }
+      asm volatile("fence.proxy.async;" ::: "memory");  // acquired peer data -> visible to the bulk loads
+      const unsigned char* uin = p.u[in];
+      unsigned char* uout = p.u[out];
+      const unsigned char* lo_src = p.left_u[in] + static_cast<size_t>(R - d) * p.row_bytes;
+      const unsigned char* hi_src = p.right_u[in];
+      const int n_in = R + 2 * d;  // input tiles of a column
+      const uint64_t loads = ncols * static_cast<uint64_t>(n_in);
+      const uint64_t events = ncols * static_cast<uint64_t>(n_in - 2);
+      uint64_t issued = 0, retired = 0;  // tiles of THIS sweep, in load order
+      size_t jj_l = 0;                   // load cursor: column tile, input tile m_l (row m_l - d)
+      int m_l = 0;
+      auto issue_next = [&]() {
+        const size_t off = col_off(jj_l);
+        const uint32_t len = col_len(off);
+        const unsigned char* src = m_l < d       ? lo_src + static_cast<size_t>(m_l) * p.row_bytes + off
+                                   : m_l < R + d ? uin + static_cast<size_t>(m_l - d) * p.row_bytes + off
+                                                 : hi_src + static_cast<size_t>(m_l - R - d) * p.row_bytes + off;
+        ptx::mbar_arrive_expect_tx(&full[ld.slot], len);
+        ptx::bulk_g2s(smem + static_cast<size_t>(ld.slot) * T, src, len, &full[ld.slot]);
+        ld.advance(1, S);
+        ++issued;
+        if (++m_l == n_in) {
+          m_l = 0;
+          ++jj_l;
+        }
+      };
+      size_t jj_c = 0;     // event cursor: column tile, arrival i
+      int i = 2;
+      uint64_t t = 0;      // tile (in load order) of the current event
+      bool pending = false;  // a store newer than the last bulk_wait_read<0> may still read its slot
+      for (uint64_t e = 0; e < events; ++e) {
+        while (issued < loads && issued < retired + static_cast<uint64_t>(S)) issue_next();
+        if (!mbar_wait_or_abort(&computed[done.slot], done.phase, abort_w)) return;
+        done.advance(1, S);
+        if (i >= 2 * d) {
+          const size_t off = col_off(jj_c);
+          ptx::bulk_s2g(uout + static_cast<size_t>(i - 2 * d) * p.row_bytes + off,
+                        smem + static_cast<size_t>(ev.slot) * T, col_len(off));
+          ptx::bulk_commit();
+          ptx::bulk_wait_read<1>();  // every store but the newest has left shared memory
+          retired = t;
+          pending = true;
+        } else {
+          if (pending) ptx::bulk_wait_read<0>();
+          pending = false;
+          retired = t + 1;
+        }
+        ++t;
+        ev.advance(1, S);
+        if (++i == n_in) {  // next column: the last two input tiles are no event slot
+          i = 2;
+          ++jj_c;
+          t += 2;
+          ev.advance(2, S);
+        }
+      }
+      ptx::bulk_wait<0>();  // this sweep's stores are performed
+      asm volatile("fence.proxy.async;" ::: "memory");
+      ptx::fence_acq_rel_sys();
+      ptx::st_release_sys(p.signal_hi + blockIdx.x * kHaloFlagWords, g + static_cast<uint32_t>(d));
+      ptx::st_release_sys(p.signal_lo + blockIdx.x * kHaloFlagWords, g + static_cast<uint32_t>(d));
+      k += d;
+    }
+  } else {
+    // ------------------------------------------------------------------ math warps ----
+    constexpr int P = (kSweepMaxTileBytes / 16 + 32 * kSweepMathWarps - 1) / (32 * kSweepMathWarps);  // float4 / thread
+    const uint32_t mt = threadIdx.x - 32;
+    const float alpha = p.alpha, s = p.s;
+    // lv[L-1][0|1][k]: rows q-1, q of level L (the two newest) at position k, L = 1 .. D-1
+    float4 lv[D - 1][2][P];
+#pragma unroll
+    for (int L = 0; L < D - 1; ++L)
+#pragma unroll
+      for (int k = 0; k < P; ++k) lv[L][0][k] = lv[L][1][k] = make_float4(0.f, 0.f, 0.f, 0.f);
+    Ring up_t{0, 0};  // input tile i-2 of arrival i (overwritten with level d of row i-2d)
+    Ring done{0, 0};
+    for (int ks = 0; ks < p.steps;) {
+      const int d = sweep_depth(p.steps - ks, D);
+      const int n_in = R + 2 * d;
+      for (size_t jj = 0; jj < ncols; ++jj) {
+        const uint32_t nv = col_len(col_off(jj)) / 16;
+        for (int i = 2; i < n_in; ++i) {
+          const Ring ce_t = up_t.at(1, S), dn_t = up_t.at(2, S);
+          if (i == 2) {
+            if (!mbar_wait_or_abort(&full[up_t.slot], up_t.phase, abort_w)) return;
+            if (!mbar_wait_or_abort(&full[ce_t.slot], ce_t.phase, abort_w)) return;
+          }
+          if (!mbar_wait_or_abort(&full[dn_t.slot], dn_t.phase, abort_w)) return;
+          float4* up = reinterpret_cast<float4*>(smem + static_cast<size_t>(up_t.slot) * T);
+          const float4* ce = reinterpret_cast<const float4*>(smem + static_cast<size_t>(ce_t.slot) * T);
+          const float4* dn = reinterpret_cast<const float4*>(smem + static_cast<size_t>(dn_t.slot) * T);
+          const bool store = i >= 2 * d;
+#pragma unroll
+          for (int k = 0; k < P; ++k) {
+            const uint32_t v = mt + static_cast<uint32_t>(k) * 32 * kSweepMathWarps;
+            if (v < nv) {
+              float4 x = stencil4(up[v], ce[v], dn[v], alpha, s);  // level 1, row i-d-1
+#pragma unroll
+              for (int L = 2; L <= D; ++L) {
+                if (L <= d) {
+                  float4 y = x;  // not valid before arrival 2L, and then only feeds levels that are not valid either
+                  if (i >= 2 * L) y = stencil4(lv[L - 2][0][k], lv[L - 2][1][k], x, alpha, s);  // level L, row i-d-L
+                  lv[L - 2][0][k] = lv[L - 2][1][k];
+                  lv[L - 2][1][k] = x;
+                  x = y;
+                }
+              }
+              if (store) up[v] = x;
+            }
+          }
+          if (store) ptx::fence_proxy_async_smem();  // generic-proxy smem writes -> visible to the TMA store
+          __syncwarp();
+          if ((threadIdx.x & 31) == 0) ptx::mbar_arrive(&computed[done.slot]);
+          done.advance(1, S);
+          up_t.advance(1, S);
+        }
+        up_t.advance(2, S);
+      }
+      ks += d;
+    }
+  }
+}
+
 // ------------------------------------------------------------- field values ----
 // u0(global row, column): a hash folded to [-32, 32) with 10 fractional bits, reproducible on the host
 // (models/halo.py::initial_field).
@@ -353,9 +585,9 @@ struct HaloGeometry {
   int ctas;
 };
 
-template <int kMode>
+template <auto kKernel, int kThreads>
 int occupancy_of(size_t smem) {
-  // One attribute + occupancy query per (mode, smem, device), not per launch (per-step launches come here K times).
+  // One attribute + occupancy query per (kernel, smem, device), not per launch (per-step launches come here K times).
   // The dynamic shared-memory limit of the function is only ever RAISED: instances with different stage counts coexist.
   struct Entry {
     size_t smem;
@@ -368,15 +600,23 @@ int occupancy_of(size_t smem) {
   HPCP_CUDA(cudaGetDevice(&device));
   std::lock_guard<std::mutex> lk(mu);
   if (device >= 0 && device < 64 && smem > limit_set[device]) {
-    HPCP_ENABLE_SMEM(halo_stencil_kernel<kMode>, smem);
+    HPCP_ENABLE_SMEM(kKernel, smem);
     limit_set[device] = smem;
   }
   for (const Entry& e : cache)
     if (e.smem == smem && e.device == device) return e.per_sm;
   int per_sm = 0;
-  HPCP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, halo_stencil_kernel<kMode>, kHaloThreads, smem));
+  HPCP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kKernel, kThreads, smem));
   cache.push_back({smem, device, per_sm});
   return per_sm;
+}
+
+// Deep sweeps need pull mode, tiles of at most 16 KiB (the register state of the wavefront) and the default L2 policy
+// (the evict_first hint exists only in halo_stencil_kernel); rows do not matter here, so the grid does not depend on
+// them.
+bool sweeps_allowed(HaloMode mode, const HaloTuning& tune) {
+  const int tile_kb = tune.tile_kb > 0 ? tune.tile_kb : 16;
+  return mode == HaloMode::kPull && tune.depth != 1 && tile_kb * 1024u <= kSweepMaxTileBytes && tune.l2_hint == 0;
 }
 
 HaloGeometry halo_geometry(size_t row_bytes, const HaloTuning& tune, HaloMode mode, int device) {
@@ -390,10 +630,14 @@ HaloGeometry halo_geometry(size_t row_bytes, const HaloTuning& tune, HaloMode mo
   int per_sm = 1;
   // Co-residency: a persistent multi-step launch spins on neighbour words, so every CTA must be resident.
   switch (mode) {
-    case HaloMode::kNone: per_sm = occupancy_of<0>(g.smem); break;
-    case HaloMode::kPull: per_sm = occupancy_of<1>(g.smem); break;
-    case HaloMode::kPush: per_sm = occupancy_of<2>(g.smem); break;
+    case HaloMode::kNone: per_sm = occupancy_of<halo_stencil_kernel<0>, kHaloThreads>(g.smem); break;
+    case HaloMode::kPull: per_sm = occupancy_of<halo_stencil_kernel<1>, kHaloThreads>(g.smem); break;
+    case HaloMode::kPush: per_sm = occupancy_of<halo_stencil_kernel<2>, kHaloThreads>(g.smem); break;
   }
+  // A time series mixes single-step and deep launches with the same step words (indexed by CTA): one grid that both
+  // kernels keep fully resident.
+  if (sweeps_allowed(mode, tune))
+    per_sm = std::min(per_sm, occupancy_of<halo_sweep_kernel<3>, kSweepThreads>(g.smem));
   HPCP_REQUIRE(per_sm >= 1, "halo_stencil: kernel does not fit on an SM");
   const size_t tiles = (row_bytes + g.tile_bytes - 1) / g.tile_bytes;
   const int resident = std::min(sms * per_sm, kHaloMaxCtas);  // one step word per CTA and side
@@ -407,6 +651,24 @@ HaloGeometry halo_geometry(size_t row_bytes, const HaloTuning& tune, HaloMode mo
 
 int halo_stencil_ctas(size_t row_elems, const HaloTuning& tune, HaloMode mode, int device) {
   return halo_geometry(row_elems * sizeof(float), tune, mode, device).ctas;
+}
+
+int halo_sweep_depth(int rows, HaloMode mode, const HaloTuning& tune) {
+  HPCP_REQUIRE(tune.depth >= 0, "halo_stencil: depth >= 0");
+  if (!sweeps_allowed(mode, tune)) return 1;
+  // Halo rows come only from the immediate neighbours: depth <= rows.  Depth 3 is the only instantiation: depth 5 keeps
+  // 2 x 4 x 11 float4 = 352 registers of wavefront state per thread, more than two CTAs per SM can hold.
+  const int want = std::min(tune.depth > 0 ? tune.depth : kHaloDefaultDepth, rows);
+  return want >= 3 ? 3 : 1;
+}
+
+std::vector<int> halo_sweep_schedule(int steps, int depth) {
+  std::vector<int> out;
+  for (int k = 0; k < steps;) {
+    out.push_back(sweep_depth(steps - k, depth));
+    k += out.back();
+  }
+  return out;
 }
 
 int launch_halo_stencil(const HaloStencilArgs& a, HaloMode mode, const HaloTuning& tune, int device,
@@ -468,6 +730,34 @@ int launch_halo_stencil(const HaloStencilArgs& a, HaloMode mode, const HaloTunin
     p.wait_hi = a.flags_local + set_words + side_words;
     p.signal_lo = a.flags_left + set_words + side_words;  // I am the right neighbour of my left neighbour
     p.signal_hi = a.flags_right + set_words;              // and the left neighbour of my right neighbour
+  }
+  const int depth = halo_sweep_depth(a.rows, mode, tune);
+  if (depth > 1 && sweep_depth(a.steps, depth) > 1) {  // at least one deep sweep: K >= 4
+    SweepParams q{};
+    for (int r = 0; r < 2; ++r) {
+      q.u[r] = p.u[r];
+      q.left_u[r] = reinterpret_cast<const unsigned char*>(a.left_u[r]);
+      q.right_u[r] = reinterpret_cast<const unsigned char*>(a.right_u[r]);
+    }
+    q.wait_lo = p.wait_lo;
+    q.wait_hi = p.wait_hi;
+    q.signal_lo = p.signal_lo;
+    q.signal_hi = p.signal_hi;
+    q.rows = p.rows;
+    q.row_bytes = p.row_bytes;
+    q.tile_begin = p.tile_begin;
+    q.tile_end = p.tile_end;
+    q.tile_bytes = p.tile_bytes;
+    q.stages = p.stages;
+    q.alpha = p.alpha;
+    q.s = p.s;
+    q.step_base = p.step_base;
+    q.steps = p.steps;
+    q.timeout_ns = p.timeout_ns;
+    q.status = p.status;
+    halo_sweep_kernel<3><<<ctas, kSweepThreads, g.smem, stream>>>(q);
+    HPCP_CUDA(cudaGetLastError());
+    return ctas;
   }
   switch (mode) {
     case HaloMode::kNone: launch(halo_stencil_kernel<0>); break;

@@ -65,6 +65,7 @@ void print_help() {
                " --stock memcpy     the reference's shape through stock calls: kernel; wait; copies; wait\n"
                " --ctas N --tile-kb N --stages N   kernel geometry\n"
                " --l2-hint             evict_first L2 policy on the slab's own streaming loads / stores\n"
+               " --depth D     pull: most steps one sweep of the slab advances (0: default, 1: one step per sweep)\n"
                " --json FILE   append one JSON row\n"
                " --cpu         no GPU: ranks are host threads, the exchange is a memcpy into (push) or a read out of\n"
                "               (pull) the neighbours' arrays, one barrier per step: options, ring order, verification\n"
@@ -346,7 +347,8 @@ int main(int argc, char** argv) {
         {"ctas", required_argument, nullptr, 9}, {"tile-kb", required_argument, nullptr, 10},
         {"stages", required_argument, nullptr, 11}, {"json", required_argument, nullptr, 12},
         {"l2-hint", no_argument, nullptr, 13}, {"cpu", no_argument, nullptr, 14},
-        {"dump", required_argument, nullptr, 15}, {"help", no_argument, nullptr, 'h'}, {nullptr, 0, nullptr, 0}};
+        {"dump", required_argument, nullptr, 15}, {"depth", required_argument, nullptr, 16},
+        {"help", no_argument, nullptr, 'h'}, {nullptr, 0, nullptr, 0}};
     int opt;
     while ((opt = getopt_long(argc, argv, "hn:", long_opts, nullptr)) != -1) {
       switch (opt) {
@@ -367,6 +369,7 @@ int main(int argc, char** argv) {
         case 13: cfg.tune.l2_hint = 1; break;
         case 14: cfg.cpu = true; break;
         case 15: cfg.dump_path = optarg; break;
+        case 16: cfg.tune.depth = std::max(0, std::atoi(optarg)); break;
         default: print_help(); return 1;
       }
     }

@@ -16,13 +16,18 @@ periodic neighbour exchange with a true step-to-step dependency and no overlap a
   reads the boundary rows out of the neighbours' fields over NVLink with TMA bulk loads,
   ``push`` stores the new boundary rows into the neighbours' halo buffers with TMA bulk
   stores; per-CTA step words keep it RAW/WAR safe without any barrier or host sync, and
-  ``step(k)`` runs k steps in one persistent launch.
+  ``step(k)`` runs k steps in one persistent launch;
+* in pull mode a k-step launch advances the slab by up to ``depth`` steps per pass over it
+  (deep halos: ``depth`` rows pulled from each neighbour, the intermediate time levels kept
+  on chip), so HBM moves ~2*rows/depth rows per step instead of ~2*rows; the sweep sizes
+  follow ``sweep_schedule`` and the result is bit-identical to one step per pass.
 
 ``stock_step`` is the reference's shape through library calls (the thing to beat):
 compute kernel, host wait, ``cudaMemcpyAsync`` to the peers or NCCL send/recv, host wait.
 """
 from __future__ import annotations
 
+import os
 from typing import Dict, List, Optional
 
 import torch
@@ -50,6 +55,36 @@ def balanced_rows(hbm_gbs: float = 6567.4, nvlink_gbs: float = 706.1) -> int:
     """
     rows = (2.0 * hbm_gbs / nvlink_gbs - 2.0) / 2.0
     return max(1, int(rows))
+
+
+DEFAULT_SWEEP_DEPTH = 3       # kHaloDefaultDepth (csrc/kernels/api.h)
+SWEEP_MAX_TILE_KB = 16        # the deep kernel's register state is sized for 16 KiB tiles
+
+
+def sweep_depth(rows: int, mode: str, tune: Optional[dict] = None) -> int:
+    """Deepest sweep a multi-step launch takes (halo_sweep_depth in halo_stencil.cu): deep sweeps need pull mode, tiles
+    of at most 16 KiB and the default L2 policy; tune ``depth`` 0 / missing is the default, 1 one step per sweep; the
+    depth is at most ``rows`` (halo rows come from the immediate neighbours only) and 3 is the one instantiation."""
+    tune = tune or {}
+    depth = int(tune.get("depth") or 0)
+    if depth < 0:
+        raise ValueError("depth >= 0")
+    allowed = (mode == "pull" and depth != 1 and int(tune.get("tile_kb") or 16) <= SWEEP_MAX_TILE_KB
+               and not tune.get("l2_hint"))
+    return 3 if allowed and min(depth or DEFAULT_SWEEP_DEPTH, rows) >= 3 else 1
+
+
+def sweep_schedule(steps: int, depth: int) -> List[int]:
+    """Sweep sizes of a ``steps``-step launch whose deepest sweep is ``depth`` (halo_sweep_schedule in
+    halo_stencil.cu): greedy, the largest odd size <= min(depth, remaining - 1).  Odd sizes keep the ping-pong parity
+    of every step; the last sweep is one step, so the buffer of step g-1 holds it after the launch."""
+    out: List[int] = []
+    k = 0
+    while k < steps:
+        x = min(depth, steps - k - 1)
+        out.append(1 if x <= 1 else x - 1 + (x & 1))
+        k += out[-1]
+    return out
 
 
 def initial_field(world: int, rows: int, row_elems: int) -> torch.Tensor:
@@ -89,6 +124,8 @@ class HaloStencil:
         self.mode, self.alpha, self.s = mode, float(alpha), float(s)
         self.rows, self.row_bytes, self.row_elems = int(rows), int(message_bytes), int(message_bytes) // 4
         self.tune = dict(tune or {})
+        if "depth" not in self.tune and os.environ.get("HPCP_HALO_DEPTH"):
+            self.tune["depth"] = int(os.environ["HPCP_HALO_DEPTH"])
         self.left = (self.rank - 1) % self.world
         self.right = (self.rank + 1) % self.world
         torch.cuda.set_device(device)
@@ -104,6 +141,9 @@ class HaloStencil:
         if "ctas" in self.tune:
             self.ctas = min(self.ctas, int(self.tune["ctas"]))
         self.tune["ctas"] = self.ctas   # identical grid in every launch: flag words are indexed by CTA
+        # deepest sweep of a multi-step launch (1 in push / none mode, with rows < 3 or tune depth 1)
+        self.depth = sweep_depth(self.rows, mode, self.tune)
+        self.last_schedule: List[int] = [1]   # sweep sizes of the most recent multi-step launch
         self._flag_layout: Optional[int] = None   # None until the first step; 1 = whole rows, n = n column chunks
         self.g = 0                      # global step counter (monotonic; the flag words count with it)
         self.launches = 0
@@ -173,6 +213,8 @@ class HaloStencil:
         """``steps`` time steps, exchange included, in ONE kernel launch on the current stream."""
         self._use_layout(1)
         self.C.halo_stencil(self._args(steps), self.mode, self.tune, self.device, self._stream())
+        if steps > 1:   # per-step launches (timed as a side row) leave the traffic model of the persistent launch
+            self.last_schedule = sweep_schedule(steps, self.depth)
         self.g += steps
         self.launches += 1
 
@@ -339,10 +381,13 @@ class HaloStencil:
 
     # ---- traffic model (roofline rows) ------------------------------------------------------
     def hbm_bytes_per_step(self) -> int:
-        """Bytes this GPU's HBM serves per step: rows reads + rows writes of the slab, + the halo traffic."""
+        """Bytes this GPU's HBM serves per step: rows reads + rows writes of the slab, + the halo traffic.  Pull mode
+        averages over the sweeps of the most recent ``step(k)`` with k > 1 (one step per sweep before any): a sweep of
+        depth d reads and writes the slab once and serves the d boundary rows on each side that the neighbours pull."""
         r, b = self.rows, self.row_bytes
         if self.mode == "pull":
-            return (2 * r + 2) * b          # + the two boundary rows the neighbours read from here
+            sweeps = self.last_schedule
+            return sum((2 * r + 2 * d) * b for d in sweeps) // sum(sweeps)
         return (2 * r + 4) * b              # + two halo rows read here + two halo rows the neighbours write here
 
     def nvlink_bytes_per_step(self) -> int:
@@ -436,13 +481,16 @@ def main(argv: Optional[List[str]] = None) -> int:
     ap.add_argument("--stages", type=int, default=0)
     ap.add_argument("--ctas", type=int, default=0)
     ap.add_argument("--l2-hint", action="store_true", help="evict_first L2 policy on the slab's own streaming traffic")
+    ap.add_argument("--depth", type=int, default=0,
+                    help="pull: most steps one sweep of the slab advances (0: HPCP_HALO_DEPTH or the measured default, "
+                         "1: one step per sweep)")
     ap.add_argument("--json", default=None)
     args = ap.parse_args(argv)
     comm = Comm()
     dev = comm.device
     torch.cuda.set_device(dev)
     tune = {k: v for k, v in (("tile_kb", args.tile_kb), ("stages", args.stages), ("ctas", args.ctas),
-                              ("l2_hint", int(args.l2_hint))) if v}
+                              ("l2_hint", int(args.l2_hint)), ("depth", args.depth)) if v}
     hs = HaloStencil(comm, dev, args.bytes, args.rows, args.mode, tune=tune)
     if args.stock:
         enqueue = lambda: [hs.stock_step(args.stock) for _ in range(args.steps)]      # noqa: E731
@@ -459,12 +507,13 @@ def main(argv: Optional[List[str]] = None) -> int:
         bus = comm.world * 2 * args.bytes / (m["ms"] * 1e6)
         what = f"stock-{args.stock}" if args.stock else args.mode + ("/per-step" if args.per_step else "/persistent")
         print(f"Elapsed (max over ranks, min of {args.iters}): {m['ms'] * args.steps:.4f} ms for {args.steps} steps = "
-              f"{m['ms']:.5f} ms/step | halo {what} P={comm.world} rows={args.rows} bytes={args.bytes} ctas={hs.ctas} | "
+              f"{m['ms']:.5f} ms/step | halo {what} P={comm.world} rows={args.rows} bytes={args.bytes} ctas={hs.ctas} "
+              f"depth={hs.depth} | "
               f"{bus:.1f} GB/s P2P bus (aggregate), {bus / comm.world / 2:.1f} GB/s per GPU per direction", flush=True)
         if args.json:
             with open(args.json, "a") as f:
                 f.write(json.dumps({"pattern": "halo", "variant": what, "ranks": comm.world, "rows": args.rows,
-                                    "bytes": args.bytes, "steps": args.steps, "ms_per_step": m["ms"],
+                                    "bytes": args.bytes, "steps": args.steps, "depth": hs.depth, "ms_per_step": m["ms"],
                                     "bus_GBps": bus, "per_gpu_per_dir_GBps": bus / comm.world / 2, "ctas": hs.ctas,
                                     "mismatches": total_bad}) + "\n")
     hs.close()

@@ -1,5 +1,6 @@
 #!/usr/bin/env python
-"""Sweep the K-halo kernel's geometry (mode x tile x stages x CTAs) at the benchmark's shape; one JSON row per point.
+"""Sweep the K-halo kernel's geometry (mode x tile x stages x CTAs x sweep depth) at the benchmark's shape; one JSON row
+per point.
 
     python scripts/halo_tune.py --out gpurun_out/halo_tune.jsonl            # 1 GPU (loop-back)
     torchrun --nproc-per-node 2 scripts/halo_tune.py --out ...              # over NVLink
@@ -30,6 +31,8 @@ def main() -> int:
                     help="tile_kb x stages")
     ap.add_argument("--ctas", type=int, nargs="+", default=[0])
     ap.add_argument("--l2-hint", type=int, nargs="+", default=[0], help="0: default L2 policy, 1: evict_first streaming")
+    ap.add_argument("--depth", type=int, nargs="+", default=[0],
+                    help="pull: most steps per sweep of the slab (0: the default, 1: one step per sweep)")
     ap.add_argument("--bytes", type=int, default=REFERENCE_MESSAGE_BYTES)
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--preheat-ms", type=float, default=100.0)
@@ -38,9 +41,10 @@ def main() -> int:
     dev = comm.device
     torch.cuda.set_device(dev)
     rows_out = []
-    for rows, mode, geo, ctas, hint in itertools.product(args.rows, args.modes, args.geometry, args.ctas, args.l2_hint):
+    for rows, mode, geo, ctas, hint, depth in itertools.product(args.rows, args.modes, args.geometry, args.ctas,
+                                                                 args.l2_hint, args.depth):
         tile_kb, stages = (int(x) for x in geo.split("x"))
-        tune = {"tile_kb": tile_kb, "stages": stages, "l2_hint": hint}
+        tune = {"tile_kb": tile_kb, "stages": stages, "l2_hint": hint, "depth": depth}
         if ctas:
             tune["ctas"] = ctas
         try:
@@ -54,6 +58,7 @@ def main() -> int:
         m1 = timer.measure(lambda: [hs.step(1) for _ in range(args.steps)], args.steps, blocks=3, preheat_ms=0)
         bad = int(comm.sum(hs.verify_last_step()))
         row = {"world": comm.world, "rows": rows, "mode": mode, "tile_kb": tile_kb, "stages": stages, "l2_hint": hint, "ctas": hs.ctas,
+               "depth": hs.depth,
                "ms_per_step": round(m["ms"], 5), "blocks": m["blocks_ms"], "per_step_launch_ms": round(m1["ms"], 5),
                "hbm_GBps": round(hs.hbm_bytes_per_step() / m["ms"] / 1e6, 1),
                "nvlink_GBps_per_dir": round(hs.nvlink_bytes_per_step() / m["ms"] / 1e6, 1), "wrong_words": bad}
