@@ -418,8 +418,13 @@ class VirtualRing:
         tune = dict(tune or {})
         share = max(self.group.ranks_on(d) for d in set(self.group.devices))
         if share > 1:   # co-residency of the spinning persistent kernels that share a GPU
-            full = C.halo_stencil_ctas(message_bytes // 4, "pull" if mode == "none" else mode, tune, self.group.devices[0])
-            tune["ctas"] = max(1, min(tune.get("ctas") or full, full // share))
+            kind, dev = "pull" if mode == "none" else mode, self.group.devices[0]
+            if tune.get("ctas"):   # a requested grid stays as long as the CTAs of every rank fit on the GPU at once
+                tile_elems = (tune.get("tile_kb") or 16) * 256    # rows of HALO_MAX_CTAS tiles: the resident count
+                resident = C.halo_stencil_ctas(C.HALO_MAX_CTAS * tile_elems, kind, {**tune, "ctas": 0}, dev)
+                tune["ctas"] = max(1, min(tune["ctas"], resident // share))
+            else:
+                tune["ctas"] = max(1, C.halo_stencil_ctas(message_bytes // 4, kind, tune, dev) // share)
         fields = self.group.symmetric(2 * rows * message_bytes, zero=False)
         halos = self.group.symmetric(4 * message_bytes, zero=False)
         flags = self.group.symmetric(C.HALO_FLAG_BYTES, zero=True)
